@@ -222,6 +222,20 @@ def run_reference(args):
 # -----------------------------------------------------------------------------------------------------------------
 # GPU arm
 # -----------------------------------------------------------------------------------------------------------------
+DUMP_MAX_ENTRIES = 1 << 21     # per array: three float64 outputs stay within 48 MB
+
+
+def dump_outputs(directory, arrays):
+    """--dump-outputs: writes each array as <directory>/<name>.npy in float64. An array longer than DUMP_MAX_ENTRIES is written as its
+    entries at DUMP_MAX_ENTRIES fixed positions (sorted, drawn with seed 0), the same positions for every run of the same size."""
+    os.makedirs(directory, exist_ok=True)
+    for name, a in arrays.items():
+        a = np.ascontiguousarray(a, dtype=np.float64).reshape(-1)
+        if a.size > DUMP_MAX_ENTRIES:
+            a = a[np.sort(np.random.default_rng(0).choice(a.size, DUMP_MAX_ENTRIES, replace=False))]
+        np.save(os.path.join(directory, name + ".npy"), a)
+
+
 class ClockSampler:
     """SM clock + throttle reasons sampled DURING the timed region: NVML from a thread every 5 ms (an nvidia-smi
     subprocess needs >100 ms per sample, longer than a short timed region), nvidia-smi -lms as the fallback."""
@@ -500,6 +514,13 @@ def run_engine(args):
         peak_i8 = ctx.microbench_peak(1)
         main = timed_loop(args.condense, args.steps, True)
         ctx.sync()
+        if args.dump_outputs:
+            # what solveCompressed handed back in the last timed step; dx is column-sharded like J, dyc / dyd are replicated
+            outputs = {"dx": dx.cpu().numpy().copy(), "dyc": dyc.cpu().numpy().copy(), "dyd": dyd.cpu().numpy().copy()}
+            if world > 1:
+                parts = [None] * world
+                dist.all_gather_object(parts, outputs["dx"])
+                outputs["dx"] = np.concatenate(parts)
         kkt_resid_rel = independent_kkt_residual(torch, dist, world, T, 1.0, dx, dyc, dyd)
         # the other condensation kernel on the same workload (both modes belong in the record)
         other_name = "dmma" if main["mode"] != 0 else "oz8"
@@ -664,6 +685,8 @@ def run_engine(args):
     assert kkt_resid_rel <= 1e-8 and kkt_resid_other <= 1e-8, (kkt_resid_rel, kkt_resid_other)
     if e2e is not None:
         line["e2e"] = e2e
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, outputs)
     if world == 1 and not args.no_cpu:
         line["cpu_baseline"] = cpu_baseline(args.cpu_sample, n, m, l)
     print(json.dumps(line))
@@ -809,11 +832,12 @@ def run_mds(args):
             ms = e0.elapsed_time(e1) / steps
             launches = ctx.launch_count() - launches0
             ck = sampler.stop() if sampler else None
+            outputs = {"dx": dx.cpu().numpy().copy(), "dyc": dyc.cpu().numpy().copy(), "dyd": dyd.cpu().numpy().copy()} if args.dump_outputs else None
             step(True)      # one extra, phase-stamped step (events between the phases; not part of the timed region)
             resid = mds_independent_residual(torch, T, nxs, nxd, neq, nineq, dx, dyc, dyd)
             k.close()
             return {"ms_step": ms, "launches": launches, "clocks": ck, "phase_ms": {"assemble": phase[0], "factor+inertia": phase[1], "solve": phase[2]},
-                    "resid": resid}
+                    "resid": resid, "outputs": outputs}
 
         bk = run_mode(True, args.steps, True)
         nopiv = run_mode(False, max(3, min(args.steps, 10)), False)
@@ -840,6 +864,8 @@ def run_mds(args):
                            "roofline": roof(nopiv, "look-ahead LDL^T: k_diag128 + k_trsm_panel + k_gemm_pq<64> (FP64 DMMA)")},
             "measured_peaks_in_run": {"fp64_dmma_tflops": peak_dmma}}
     assert bk["resid"] <= 1e-8 and nopiv["resid"] <= 1e-8, (bk["resid"], nopiv["resid"])
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, bk["outputs"])
     if not args.no_cpu:
         line["cpu_baseline"] = mds_cpu_baseline(args, nnz_row)
     print(json.dumps(line))
@@ -895,7 +921,13 @@ def main():
     ap.add_argument("--mds-nd", type=int, default=20000)
     ap.add_argument("--mds-m", type=int, default=2000)
     ap.add_argument("--ref-sampled", action="store_true", help="--impl reference: report the two-sample extrapolation instead of one full-size system")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="engine arms: after the timed steps, write dx, dyc and dyd of the last timed step as DIR/<name>.npy "
+                    "(float64; arrays over 2^21 entries as a fixed, seeded sample) so that two builds can be compared output for output")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs applies to the engine arms")
     if args.impl == "reference":
         return run_reference(args)
     if args.workload == "mds":

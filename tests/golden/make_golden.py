@@ -1,8 +1,10 @@
-"""Generates tests/golden/*.npz by running the UNMODIFIED reference (oracle/_ref, built by oracle/Makefile from
-/root/reference) on seeded synthetic inputs. Run in the build container only:  python tests/golden/make_golden.py
-The fixtures freeze (inputs, reference outputs) tuples so that the GPU box -- which has no /root/reference -- can
-check both the oracle restatement and the CUDA path against what the reference itself computed."""
+"""Generates tests/golden/*.npz by running the UNMODIFIED reference (oracle/_ref, built by `make -C oracle ref` from the
+reference's sources, REF=<its checkout>) on seeded synthetic inputs:  python tests/golden/make_golden.py
+The fixtures freeze (inputs, reference outputs) tuples so that the test suite -- which does not need the reference --
+checks both the oracle restatement and the CUDA path against what the reference itself computed. The reference's outputs
+for tests/test_oracle_vs_ref.py (tests/golden/oracle_vs_ref.npz) are recorded by that module itself."""
 import os
+import subprocess
 import sys
 
 import numpy as np
@@ -179,3 +181,5 @@ if __name__ == "__main__":
     iajaaa_case()
     vec_cases()
     mds_case()
+    subprocess.check_call([sys.executable, "-m", "pytest", "-q", "-p", "no:cacheprovider", os.path.join(ROOT, "tests", "test_oracle_vs_ref.py")],
+                          cwd=ROOT, env=dict(os.environ, HB_RECORD_REFERENCE="1"))
