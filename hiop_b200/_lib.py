@@ -61,6 +61,7 @@ def lib() -> ctypes.CDLL:
     f("hb_ctx_device", c_i, c_vp)
     f("hb_ctx_enable_timing", c_i, c_vp, c_i)
     f("hb_ctx_last_syrk_ms", c_i, c_vp, P(ctypes.c_float))
+    f("hb_ctx_set_oz_workspace_limit", c_i, c_vp, ctypes.c_size_t)
     f("hb_malloc", c_i, c_vp, ctypes.c_size_t, P(c_vp))
     f("hb_free", c_i, c_vp, c_vp)
     f("hb_malloc_host", c_i, c_vp, ctypes.c_size_t, P(c_vp))
@@ -132,6 +133,7 @@ def lib() -> ctypes.CDLL:
     f("hb_lowrank_condense_async", c_i, c_vp)
     f("hb_lowrank_check", c_i, c_vp)
     f("hb_lowrank_fallback_count", c_i, c_vp)
+    f("hb_lowrank_last_condense_chunks", c_i, c_vp)
     f("hb_lowrank_set_condense_mode", c_i, c_vp, c_i)
     f("hb_lowrank_get_condense_mode", c_i, c_vp)
     f("hb_lowrank_solve_compressed", c_i, c_vp, *([c_dp] * 6))

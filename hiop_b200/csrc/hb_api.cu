@@ -1,6 +1,7 @@
 // Context, memory and communicator plumbing of libhiopb200.so.
 #include "hb_common.cuh"
 
+#include <cstdlib>
 #include <dlfcn.h>
 
 thread_local char g_hb_err[512] = "";
@@ -32,6 +33,7 @@ extern "C" int hb_ctx_create(int device, hb_ctx** out)
   hb_ctx* c = new hb_ctx;
   c->device = device;
   c->num_sms = prop.multiProcessorCount;
+  if(const char* e = getenv("HB_OZ_WORKSPACE_MB")) c->oz_ws_limit = (size_t)strtoull(e, nullptr, 10) << 20;
   HB_CUDA(cudaStreamCreateWithFlags(&c->stream, cudaStreamNonBlocking));
   HB_CUDA(cudaMalloc(&c->red_dev, sizeof(double) * HB_RED_SLOTS));
   HB_CUDA(cudaMallocHost(&c->red_host, sizeof(double) * 64));
@@ -79,7 +81,9 @@ extern "C" int hb_ctx_last_syrk_ms(hb_ctx* c, float* ms)
 // solve_compressed; hb_ctx_phase_timeline(ctx, 0, ms) waits for them and returns the phase durations (ms) in the order
 // update, row maxima (+ fused row dots), slicing, GEMM + fix-up [= C_aug; the first two only with the int8-slice kernel, otherwise the whole
 // condensation is in the third], all-reduce, V/U/N assembly, Cholesky, H^-1 rx, J dx (+ all-reduce), SPD solve, J^T dy, H^-1 rx (second).
-// A mark that was not passed contributes 0 and its time is counted in the next recorded phase.
+// A mark that was not passed contributes 0 and its time is counted in the next recorded phase. When the int8 slices are made and
+// multiplied in several column chunks (hb_lowrank_last_condense_chunks > 1) the slicing entry is 0 and the GEMM entry holds the
+// slicing and the GEMM of all chunks.
 extern "C" int hb_ctx_phase_timeline(hb_ctx* c, int on, float* ms_host10)
 {
   HB_REQUIRE(c, "null ctx");

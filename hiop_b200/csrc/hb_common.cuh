@@ -76,6 +76,7 @@ struct hb_ctx
   // per-context state of the int8-slice condensation (hb_ozaki.cu): slice buffer, exponents, tensor maps, work list
   void* oz_state = nullptr;
   void (*oz_free)(void*) = nullptr;
+  size_t oz_ws_limit = 0; // bytes of int8 slices the condensation may hold (hb_ctx_set_oz_workspace_limit); 0 = AUTO
   // NCCL
   void* nccl_comm = nullptr;
   int nranks = 1, rank = 0;

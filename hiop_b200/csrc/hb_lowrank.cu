@@ -8,7 +8,7 @@
 
 int hb_syrk_rows(hb_ctx* c, int M, long long K, const double* const* rowptr_dev, bool aligned16, const double* d, double* C, int ldc);
 int hb_syrk_rows_ozaki(hb_ctx* c, int M, long long K, const double* const* rowptr_dev, bool rows_aligned16, const double* d, double* C, int ldc, int S,
-                       const double* dot_x, double* dot_out);
+                       const double* dot_x, double* dot_out, int* chunks_out);
 
 namespace {
 
@@ -523,7 +523,13 @@ int do_condense_async(hb_lowrank* k, const double* fuse_rx = nullptr)
     HB_CHECK(resolve_global_n(k));
     mode = (k->n_global >= 32768 && Ma >= 64) ? 8 : 0;
   }
-  HB_CHECK(condense_enqueue(k, mode, fuse_rx));
+  int rc = condense_enqueue(k, mode, fuse_rx);
+  if(rc == HB_ERR_ALLOC && k->condense_mode < 0 && mode != 0) {
+    // not even one column chunk of int8 slices fits the slice budget: the FP64 kernel needs no slice buffer
+    k->fallbacks++;
+    rc = condense_enqueue(k, 0, fuse_rx);
+  }
+  HB_CHECK(rc);
   k->check_pending = true;
   k->cond_valid = true; // optimistic: a failure is reported by the next synchronous call (hb_lowrank_check / hb_lowrank_condense)
   return HB_OK;
@@ -574,11 +580,13 @@ int condense_enqueue(hb_lowrank* k, int mode, const double* fuse_rx)
   k->tdot_valid = false;
   if(Ma > 0) {
     k->condense_used = mode;
+    k->condense_chunks = 0;
     if(mode == 0) HB_CHECK(hb_syrk_rows(c, Ma, k->n, k->rowptr_dev, k->rows_aligned, k->DhInv, k->Caug, Ma));
     else {
       const bool fuse = fuse_rx && m > 0;
       if(fuse && k->n == 0) HB_CUDA(cudaMemsetAsync(k->tdot, 0, sizeof(double) * Ma, c->stream));
-      HB_CHECK(hb_syrk_rows_ozaki(c, Ma, k->n, k->rowptr_dev, k->rows_aligned, k->DhInv, k->Caug, Ma, mode, fuse ? fuse_rx : nullptr, fuse ? k->tdot : nullptr));
+      HB_CHECK(hb_syrk_rows_ozaki(c, Ma, k->n, k->rowptr_dev, k->rows_aligned, k->DhInv, k->Caug, Ma, mode, fuse ? fuse_rx : nullptr, fuse ? k->tdot : nullptr,
+                                  &k->condense_chunks));
       k->tdot_valid = fuse;
     }
   }
@@ -816,6 +824,7 @@ extern "C" int hb_lowrank_check(hb_lowrank* k)
   return condense_check(k);
 }
 extern "C" int hb_lowrank_fallback_count(hb_lowrank* k) { return k ? k->fallbacks : 0; }
+extern "C" int hb_lowrank_last_condense_chunks(hb_lowrank* k) { return k ? k->condense_chunks : 0; }
 
 extern "C" int hb_lowrank_hess_solve(hb_lowrank* k, const double* rhs, double* x)
 {

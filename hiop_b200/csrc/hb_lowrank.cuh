@@ -30,7 +30,8 @@ struct hb_lowrank
   int condense_used = 0;
   long long n_global = -1; // sum of n over the ranks (the auto rule must not depend on the world size); resolved at the first condensation
   bool check_pending = false; // an asynchronous condensation left its info words unchecked
-  int fallbacks = 0;          // times the FP64 kernel had to redo an int8-slice condensation whose Cholesky broke down
+  int fallbacks = 0;          // AUTO-mode condensations the FP64 kernel redid: the int8-slice Cholesky broke down or its slices did not fit
+  int condense_chunks = 0;    // column chunks of the last int8-slice condensation (1 = unchunked); 0 = the FP64 kernel ran
   double* tri = nullptr;      // packed upper triangle of C_aug for the all-reduce
   double* tdot = nullptr;     // [J; S; Y] (DhInv .* rx) from the fused row-maximum sweep of an int8-slice condensation (m + 2 lmax)
   bool tdot_valid = false;

@@ -14,7 +14,7 @@
 
 int hb_syrk_rows(hb_ctx* c, int M, long long K, const double* const* rowptr_dev, bool aligned16, const double* d, double* C, int ldc);
 int hb_syrk_rows_ozaki(hb_ctx* c, int M, long long K, const double* const* rowptr_dev, bool rows_aligned16, const double* d, double* C, int ldc, int S,
-                       const double* dot_x, double* dot_out);
+                       const double* dot_x, double* dot_out, int* chunks_out);
 
 namespace {
 constexpr int ET = 256;
@@ -64,7 +64,7 @@ extern "C" int hb_lowrank_lsq_duals(hb_lowrank* k, const double* grad_f, const d
     mode = (ng >= 32768 && m >= 64) ? 8 : 0;
   }
   if(mode == 0) HB_CHECK(hb_syrk_rows(c, m, n, k->rowptr_dev, k->rows_aligned, nullptr, M, m));
-  else HB_CHECK(hb_syrk_rows_ozaki(c, m, n, k->rowptr_dev, k->rows_aligned, nullptr, M, m, mode, nullptr, nullptr));
+  else HB_CHECK(hb_syrk_rows_ozaki(c, m, n, k->rowptr_dev, k->rows_aligned, nullptr, M, m, mode, nullptr, nullptr, nullptr));
   HB_CHECK(hb_allreduce_sum(c, M, (long long)m * m));
   // rhs = -J vecx (all-reduced), then the d-side terms on the replicated part
   if(n > 0) {

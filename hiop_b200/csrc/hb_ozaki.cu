@@ -17,6 +17,8 @@
 //   warps 4-7          epilogue: at every K-chunk boundary tcgen05.ld the S accumulators, recombine them in FP64 and
 //                      accumulate into the CTA's FP64 partial tile (workspace, L2 resident)
 // A last kernel sums the split-K partials in fixed order, applies 2^{e_i+e_j} and mirrors the tile (deterministic).
+// When the slices of all K columns do not fit the slice budget, K is sliced and multiplied in column chunks that reuse one buffer, the
+// GEMM of every chunk after the first adding to the partial tiles (see hb_syrk_rows_ozaki).
 #include "hb_common.cuh"
 #include <cuda.h>
 #include <cstdlib>
@@ -28,6 +30,8 @@ constexpr int KS = 128;           // bytes of K per block (one SWIZZLE_128B row 
 constexpr int A_TILE = TM * KS;   // 16 KB per slice
 constexpr int B_TILE = TN * KS;   // 8 KB per slice
 constexpr int OZ_THREADS = 256;
+// device memory the AUTO slice budget leaves free: the split-K partial tiles (<= 1 GB by the split rule) and the small buffers
+constexpr size_t OZ_FREE_MARGIN = (size_t)1 << 30;
 
 __device__ __forceinline__ uint32_t s2u(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
 __device__ __forceinline__ void mbar_init(unsigned long long* b, unsigned c) { asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;\n" ::"r"(s2u(b)), "r"(c)); }
@@ -212,8 +216,10 @@ __global__ void k_sqrt(long long n, const double* __restrict__ d, double* __rest
   for(long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += stride) sd[i] = sqrt(d[i]);
 }
 
-// Q[p][row][k] (int8, row pitch Kpad bytes, slice pitch Mpad*Kpad). One thread = 8 consecutive k of one row: a warp reads
-// 2 KB of the FP64 row with 16-byte loads and writes 256 contiguous bytes per slice.
+// Q[p][row][k - k0] (int8, row pitch ldq bytes, slice pitch Mpad*ldq) for the column window [k0, k0 + Kw), zero-padded up to
+// Kwpad (a multiple of KS). One thread = 8 consecutive k of one row: a warp reads 2 KB of the FP64 row with 16-byte loads and writes
+// 256 contiguous bytes per slice. The digits depend only on a_ik, sd_k and the row exponent e_i, so a window of a column-chunked
+// condensation holds exactly the bytes the one-window (unchunked) call writes for those columns.
 //
 // Digits without the conversion pipe: with b = a*sd / 2^e (|b| < 1), hi = rint(b * 2^27) carries the first four slices
 // (6+7+7+7 bits) and lo = rint((b*2^27 - hi) * 2^(7(S-4))) the remaining S-4. Both roundings use the 1.5*2^52 magic-number
@@ -233,8 +239,8 @@ __device__ __forceinline__ void oz_digits(int v, int (&d)[ND])
 }
 template <int S>
 __global__ void __launch_bounds__(256)
-k_oz_slice(const double* const* __restrict__ rowptr, int M, int Mpad, long long K, long long Kpad, const double* __restrict__ sd,
-           const int* __restrict__ e, int8_t* __restrict__ Q, int vec_ok)
+k_oz_slice(const double* const* __restrict__ rowptr, int M, int Mpad, long long kwin, long long K, long long Kpad, long long ldq,
+           const double* __restrict__ sd, const int* __restrict__ e, int8_t* __restrict__ Q, int vec_ok)
 {
   static_assert(S >= 5 && S <= 8, "slices");
   constexpr int NLO = S - 4;
@@ -244,8 +250,9 @@ k_oz_slice(const double* const* __restrict__ rowptr, int M, int Mpad, long long 
   double x[8];
 #pragma unroll
   for(int j = 0; j < 8; j++) x[j] = 0.0;
+  if(sd) sd += kwin; // kwin is a multiple of KS: 16-byte alignment of the rows and of sd is kept
   if(row < M) {
-    const double* a = rowptr[row];
+    const double* a = rowptr[row] + kwin;
     const double sc = ldexp(1.0, 27 - e[row]);
     if(vec_ok && k0 + 7 < K) {
 #pragma unroll
@@ -285,7 +292,7 @@ k_oz_slice(const double* const* __restrict__ rowptr, int M, int Mpad, long long 
       w[4 + p][h] = __byte_perm(__byte_perm(dl[0][p], dl[1][p], 0x0040), __byte_perm(dl[2][p], dl[3][p], 0x0040), 0x5410);
   }
 #pragma unroll
-  for(int p = 0; p < S; p++) *reinterpret_cast<uint2*>(Q + ((size_t)p * Mpad + row) * Kpad + k0) = make_uint2(w[p][0], w[p][1]);
+  for(int p = 0; p < S; p++) *reinterpret_cast<uint2*>(Q + ((size_t)p * Mpad + row) * ldq + k0) = make_uint2(w[p][0], w[p][1]);
 }
 
 // ---------------------------------------------------------------------------------------------------------------------
@@ -314,7 +321,7 @@ struct OzCfg
 template <int S>
 __global__ void __launch_bounds__(OZ_THREADS, 1)
 k_oz_gemm(const __grid_constant__ CUtensorMap mapA, const __grid_constant__ CUtensorMap mapB, const OzItem* __restrict__ items, int n_items,
-          int chunk_blocks, double* __restrict__ partial)
+          int chunk_blocks, int accumulate, double* __restrict__ partial)
 {
   using Cfg = OzCfg<S>;
   constexpr int RING = Cfg::RING;
@@ -444,7 +451,7 @@ k_oz_gemm(const __grid_constant__ CUtensorMap mapA, const __grid_constant__ CUte
         asm volatile("tcgen05.fence::before_thread_sync;\n" ::: "memory");
         __syncwarp();
         if(lane == 0) mbar_arrive(accempty);
-        if(c == 0) {
+        if(c == 0 && !accumulate) {
 #pragma unroll
           for(int j = 0; j < TN; j += 2) *reinterpret_cast<double2*>(slot + j) = make_double2(acc[j], acc[j + 1]);
         } else {
@@ -491,8 +498,9 @@ struct OzState
 {
   int M = -1, S = 0, splits = 0, n_tiles = 0, n_items = 0;
   long long K = -1, Kpad = 0;
+  long long Kc = 0;  // columns per slicing chunk (Kpad: unchunked); row pitch of Q
   int Mpad = 0;
-  int8_t* Q = nullptr;
+  int8_t* Q = nullptr; // S x Mpad x Kc int8 slices of the current column chunk
   size_t Qbytes = 0;
   double* sd = nullptr;
   long long sd_n = 0;
@@ -501,7 +509,7 @@ struct OzState
   int mcap = 0;
   double* dot_partial = nullptr; // [chunks][M] partial row dots of the fused row-maximum pass
   size_t dot_cap = 0;
-  OzItem* d_items = nullptr;
+  OzItem* d_items = nullptr; // 2 x n_items: the work list of a full chunk, then that of the (possibly shorter) last chunk
   int2* d_tiles = nullptr;
   CUtensorMap mapA, mapB;
 };
@@ -523,7 +531,7 @@ OzState& oz_state(hb_ctx* c)
 }
 
 template <int S>
-int launch_gemm(hb_ctx* c, OzState& st, int chunk_blocks, double* partial)
+int launch_gemm(hb_ctx* c, OzState& st, const OzItem* items, int chunk_blocks, int accumulate, double* partial)
 {
   const size_t smem = OzCfg<S>::SMEM;
   static bool attr[16] = {false}; // function attributes are per device
@@ -532,19 +540,46 @@ int launch_gemm(hb_ctx* c, OzState& st, int chunk_blocks, double* partial)
     if(c->device < 16) attr[c->device] = true;
   }
   const int G = st.n_items < c->num_sms ? st.n_items : c->num_sms;
-  k_oz_gemm<S><<<G, OZ_THREADS, smem, c->stream>>>(st.mapA, st.mapB, st.d_items, st.n_items, chunk_blocks, partial);
+  k_oz_gemm<S><<<G, OZ_THREADS, smem, c->stream>>>(st.mapA, st.mapB, items, st.n_items, chunk_blocks, accumulate, partial);
   HB_LAUNCHED();
   return HB_OK;
 }
 
 } // namespace
 
+// Explicit bound on the int8 slice buffer (0 = AUTO). A buffer held above the new bound is released now.
+extern "C" int hb_ctx_set_oz_workspace_limit(hb_ctx* c, size_t bytes)
+{
+  HB_REQUIRE(c, "null ctx");
+  c->oz_ws_limit = bytes;
+  if(bytes && c->oz_state) {
+    OzState& st = oz_state(c);
+    if(st.Qbytes > bytes) {
+      HB_CUDA(cudaStreamSynchronize(c->stream));
+      HB_CUDA(cudaFree(st.Q));
+      st.Q = nullptr;
+      st.Qbytes = 0;
+      st.M = -1; // the tensor maps pointed into the released buffer
+    }
+  }
+  return HB_OK;
+}
+
 // Same contract as hb_syrk_rows (C = A diag(d) A^T, both triangles), computed with S int8 slices on tcgen05.
 // dot_x/dot_out (optional, device): dot_out[i] = sum_k row_i[k] d[k] dot_x[k] over the local columns, produced by the row-maximum pass
+// chunks_out (optional, host): how many column chunks were sliced (1 = the whole of K at once)
+//
+// Column chunks. The slice buffer of all K columns (S * Mpad * Kpad bytes, as large as A in FP64 at S = 8) is allocated when it fits
+// the budget: hb_ctx_set_oz_workspace_limit / HB_OZ_WORKSPACE_MB, or, without one, the free device memory minus OZ_FREE_MARGIN.
+// Otherwise K is cut into chunks of a whole number of int32-safe recombination chunks (chunk_stages * KS columns) and each chunk is
+// sliced into a buffer of S * Mpad * Kc bytes and multiplied in turn; the first GEMM writes the FP64 partial tiles, the later ones add
+// to them. The row exponents come from one sweep over all columns first, so every digit is the one the unchunked call makes; only the
+// grouping of the FP64 partial sums changes. HB_ERR_ALLOC when not even one recombination chunk (or all of K, if smaller) fits.
 int hb_syrk_rows_ozaki(hb_ctx* c, int M, long long K, const double* const* rowptr_dev, bool rows_aligned16, const double* d, double* C, int ldc, int S,
-                       const double* dot_x, double* dot_out)
+                       const double* dot_x, double* dot_out, int* chunks_out)
 {
   HB_REQUIRE(c && M >= 0 && K >= 0 && ldc >= M && (S == 6 || S == 7 || S == 8), "hb_syrk_rows_ozaki: bad arguments");
+  if(chunks_out) *chunks_out = 1;
   if(M == 0) return HB_OK;
   if(K == 0) {
     HB_CUDA(cudaMemset2DAsync(C, sizeof(double) * ldc, 0, sizeof(double) * M, M, c->stream));
@@ -558,7 +593,33 @@ int hb_syrk_rows_ozaki(hb_ctx* c, int M, long long K, const double* const* rowpt
   OzState& st = oz_state(c);
   const int Mpad = ((M + TM - 1) / TM) * TM;
   const long long Kpad = ((K + KS - 1) / KS) * KS;
-  const size_t qbytes = (size_t)S * Mpad * Kpad;
+  // (t+1) * Kc * 2^12 < 2^31 with t+1 <= S  ->  Kc <= 2^19 / S columns
+  int chunk_stages = (int)((524288 / S) / KS);
+  // strict: S products of |q q'| <= 2^12 per column must stay BELOW 2^31 (S = 8 gives exactly 2^31 with 512 stages of 128 columns when
+  // every digit is -64, see tests/test_cpu_oz_model.py)
+  while((long long)S * chunk_stages * KS * 4096 >= (1LL << 31)) chunk_stages--;
+  // column chunk width: all of K when its slices are already held or fit the budget, else the most recombination chunks that fit
+  long long Kc = Kpad;
+  if(st.Qbytes < (size_t)S * Mpad * Kpad) {
+    size_t budget = c->oz_ws_limit;
+    if(!budget) {
+      size_t free_b = 0, total_b = 0;
+      HB_CUDA(cudaMemGetInfo(&free_b, &total_b));
+      budget = st.Qbytes + (free_b > OZ_FREE_MARGIN ? free_b - OZ_FREE_MARGIN : 0);
+    }
+    if((size_t)S * Mpad * Kpad > budget) {
+      const long long rcols = (long long)chunk_stages * KS;
+      const long long nr = (long long)(budget / ((size_t)S * Mpad * rcols));
+      if(nr == 0 || Kpad <= rcols) {
+        const long long minc = Kpad < rcols ? Kpad : rcols;
+        snprintf(g_hb_err, sizeof(g_hb_err), "hb_syrk_rows_ozaki: the int8 slices of one %lld-column chunk (%llu bytes) exceed the %llu-byte budget",
+                 minc, (unsigned long long)S * Mpad * minc, (unsigned long long)budget);
+        return HB_ERR_ALLOC;
+      }
+      Kc = nr * rcols;
+    }
+  }
+  const size_t qbytes = (size_t)S * Mpad * Kc;
   if(st.Qbytes < qbytes) {
     HB_CUDA(cudaStreamSynchronize(c->stream));
     cudaFree(st.Q);
@@ -567,6 +628,8 @@ int hb_syrk_rows_ozaki(hb_ctx* c, int M, long long K, const double* const* rowpt
     st.Qbytes = qbytes;
     st.M = -1;
   }
+  const int ncc = (int)((Kpad + Kc - 1) / Kc); // column chunks
+  if(chunks_out) *chunks_out = ncc;
   if(st.sd_n < K) {
     HB_CUDA(cudaStreamSynchronize(c->stream));
     cudaFree(st.sd);
@@ -580,8 +643,9 @@ int hb_syrk_rows_ozaki(hb_ctx* c, int M, long long K, const double* const* rowpt
     HB_CUDA(cudaMalloc(&st.e, sizeof(int) * Mpad));
     st.mcap = Mpad;
   }
-  if(st.M != M || st.K != K || st.S != S) {
-    // schedule: tiles (bi, bj) with bj >= 2 bi cover the upper triangle; split K so that ~all SMs get one item
+  if(st.M != M || st.K != K || st.S != S || st.Kc != Kc) {
+    // schedule: tiles (bi, bj) with bj >= 2 bi cover the upper triangle; split the K stages of one column chunk so that ~all SMs get one
+    // item (unchunked: the chunk is all of K)
     HB_CUDA(cudaStreamSynchronize(c->stream));
     const int nbi = Mpad / TM, nbj = Mpad / TN;
     std::vector<int2> tiles;
@@ -589,7 +653,7 @@ int hb_syrk_rows_ozaki(hb_ctx* c, int M, long long K, const double* const* rowpt
       for(int bj = 2 * bi; bj < nbj; bj++)
         if(bj * TN < M) tiles.push_back(make_int2(bi, bj));
     const int nt = (int)tiles.size();
-    const long long kstages = Kpad / KS;
+    const long long kstages = Kc / KS;
     // K splits. Default: one wave, splits = SMs / tiles (every CTA gets one item; 72 tiles x 2 splits = 144 of 148 SMs at m = 1000).
     // Where that leaves the machine badly filled (81 tiles at m = 1024: one split, 81 of 148 SMs busy) several waves of the persistent
     // CTAs are considered: the makespan is ceil(tiles * splits / SMs) / splits of one tile's full-K time, e.g. 9 splits = 729 items = 4.9
@@ -614,33 +678,37 @@ int hb_syrk_rows_ozaki(hb_ctx* c, int M, long long K, const double* const* rowpt
       }
     }
     if(splits > kstages) splits = (int)(kstages > 0 ? kstages : 1);
+    // the same tile x split list and slots for every chunk; the last chunk may be shorter (items with k_count = 0 do nothing)
+    const long long last_stages = (Kpad - (long long)(ncc - 1) * Kc) / KS;
     std::vector<OzItem> items;
-    // split-major order: the CTAs of one split sweep the same K range concurrently (operand reuse in L2)
-    for(int s = 0; s < splits; s++)
-      for(int t = 0; t < nt; t++) {
-        OzItem it;
-        it.bi = tiles[t].x; it.bj = tiles[t].y;
-        const long long b = hb_part_begin(kstages, splits, s), e2 = hb_part_begin(kstages, splits, s + 1);
-        it.k_begin = (int)b; it.k_count = (int)(e2 - b);
-        it.slot = t * splits + s;
-        items.push_back(it);
-      }
+    for(long long cst : {kstages, last_stages})
+      // split-major order: the CTAs of one split sweep the same K range concurrently (operand reuse in L2)
+      for(int s = 0; s < splits; s++)
+        for(int t = 0; t < nt; t++) {
+          OzItem it;
+          it.bi = tiles[t].x; it.bj = tiles[t].y;
+          const long long b = hb_part_begin(cst, splits, s), e2 = hb_part_begin(cst, splits, s + 1);
+          it.k_begin = (int)b; it.k_count = (int)(e2 - b);
+          it.slot = t * splits + s;
+          items.push_back(it);
+        }
     cudaFree(st.d_items); cudaFree(st.d_tiles);
     HB_CUDA(cudaMalloc(&st.d_items, sizeof(OzItem) * items.size()));
     HB_CUDA(cudaMalloc(&st.d_tiles, sizeof(int2) * nt));
     HB_CUDA(cudaMemcpy(st.d_items, items.data(), sizeof(OzItem) * items.size(), cudaMemcpyHostToDevice));
     HB_CUDA(cudaMemcpy(st.d_tiles, tiles.data(), sizeof(int2) * nt, cudaMemcpyHostToDevice));
-    cuuint64_t dims[3] = {(cuuint64_t)Kpad, (cuuint64_t)Mpad, (cuuint64_t)S};
-    cuuint64_t strides[2] = {(cuuint64_t)Kpad, (cuuint64_t)Kpad * Mpad};
+    // the maps describe the chunk buffer (row pitch Kc); every chunk is sliced into the same buffer, so they stay valid
+    cuuint64_t dims[3] = {(cuuint64_t)Kc, (cuuint64_t)Mpad, (cuuint64_t)S};
+    cuuint64_t strides[2] = {(cuuint64_t)Kc, (cuuint64_t)Kc * Mpad};
     cuuint32_t boxA[3] = {KS, TM, 1}, boxB[3] = {KS, TN, (cuuint32_t)S}, es[3] = {1, 1, 1};
     CUresult r1 = g_encode(&st.mapA, CU_TENSOR_MAP_DATA_TYPE_UINT8, 3, st.Q, dims, strides, boxA, es, CU_TENSOR_MAP_INTERLEAVE_NONE,
                            CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
     CUresult r2 = g_encode(&st.mapB, CU_TENSOR_MAP_DATA_TYPE_UINT8, 3, st.Q, dims, strides, boxB, es, CU_TENSOR_MAP_INTERLEAVE_NONE,
                            CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
     if(r1 != CUDA_SUCCESS || r2 != CUDA_SUCCESS) return hb_fail(HB_ERR_CUDA, "cuTensorMapEncodeTiled failed%s", "");
-    st.M = M; st.K = K; st.S = S; st.Mpad = Mpad; st.Kpad = Kpad; st.splits = splits; st.n_tiles = nt; st.n_items = (int)items.size();
+    st.M = M; st.K = K; st.S = S; st.Mpad = Mpad; st.Kpad = Kpad; st.Kc = Kc; st.splits = splits; st.n_tiles = nt; st.n_items = nt * splits;
   }
-  // 1. sqrt(d), row maxima, exponents, slices
+  // 1. sqrt(d), row maxima and exponents over all K columns
   const double* sd = nullptr;
   if(d) {
     k_sqrt<<<c->num_sms * 8, 256, 0, c->stream>>>(K, d, st.sd);
@@ -677,25 +745,31 @@ int hb_syrk_rows_ozaki(hb_ctx* c, int M, long long K, const double* const* rowpt
     k_oz_exponents<<<(Mpad + 127) / 128, 128, 0, c->stream>>>(M, st.mx, st.e);
     HB_LAUNCHED();
     hb_phase_mark(c, HB_PH_OZ_ROWMAX);
-    const unsigned sx = (unsigned)((Kpad / 8 + 255) / 256);
-    const int vec_ok = rows_aligned16 ? 1 : 0;
-    if(S == 6) k_oz_slice<6><<<dim3(sx, Mpad), 256, 0, c->stream>>>(rowptr_dev, M, Mpad, K, Kpad, sd, st.e, st.Q, vec_ok);
-    else if(S == 7) k_oz_slice<7><<<dim3(sx, Mpad), 256, 0, c->stream>>>(rowptr_dev, M, Mpad, K, Kpad, sd, st.e, st.Q, vec_ok);
-    else k_oz_slice<8><<<dim3(sx, Mpad), 256, 0, c->stream>>>(rowptr_dev, M, Mpad, K, Kpad, sd, st.e, st.Q, vec_ok);
-    HB_LAUNCHED();
-    hb_phase_mark(c, HB_PH_OZ_SLICE);
   }
-  // 2. tcgen05 GEMM into FP64 partial tiles
-  HB_CHECK(hb_ws_reserve(c, sizeof(double) * (size_t)st.n_items * TM * TN));
-  // (t+1) * Kc * 2^12 < 2^31 with t+1 <= S  ->  Kc <= 2^19 / S columns
-  int chunk_stages = (int)((524288 / S) / KS);
-  // strict: S products of |q q'| <= 2^12 per column must stay BELOW 2^31 (S = 8 gives exactly 2^31 with 512 stages of 128 columns when
-  // every digit is -64, see tests/test_cpu_oz_model.py)
-  while((long long)S * chunk_stages * KS * 4096 >= (1LL << 31)) chunk_stages--;
-  if(c->timing) HB_CUDA(cudaEventRecord(c->ev_syrk0, c->stream));
-  if(S == 6) HB_CHECK(launch_gemm<6>(c, st, chunk_stages, (double*)c->ws));
-  else if(S == 7) HB_CHECK(launch_gemm<7>(c, st, chunk_stages, (double*)c->ws));
-  else HB_CHECK(launch_gemm<8>(c, st, chunk_stages, (double*)c->ws));
+  // 2. per column chunk: slices, then the tcgen05 GEMM into the FP64 partial tiles (the first chunk writes them, the later ones add)
+  const int vec_ok = rows_aligned16 ? 1 : 0;
+  // timed window (hb_ctx_last_syrk_ms): the GEMM; in chunked mode the slicing and GEMMs of all chunks
+  if(c->timing && ncc > 1) HB_CUDA(cudaEventRecord(c->ev_syrk0, c->stream));
+  for(int q = 0; q < ncc; q++) {
+    const long long k0 = (long long)q * Kc;
+    const long long kw = (K - k0 < Kc) ? K - k0 : Kc;
+    const long long kwpad = ((kw + KS - 1) / KS) * KS;
+    const unsigned sx = (unsigned)((kwpad / 8 + 255) / 256);
+    if(S == 6) k_oz_slice<6><<<dim3(sx, Mpad), 256, 0, c->stream>>>(rowptr_dev, M, Mpad, k0, kw, kwpad, Kc, sd, st.e, st.Q, vec_ok);
+    else if(S == 7) k_oz_slice<7><<<dim3(sx, Mpad), 256, 0, c->stream>>>(rowptr_dev, M, Mpad, k0, kw, kwpad, Kc, sd, st.e, st.Q, vec_ok);
+    else k_oz_slice<8><<<dim3(sx, Mpad), 256, 0, c->stream>>>(rowptr_dev, M, Mpad, k0, kw, kwpad, Kc, sd, st.e, st.Q, vec_ok);
+    HB_LAUNCHED();
+    if(q == 0) {
+      // the slicing phase mark only when the slicing is one phase; in chunked mode the slicing counts under the GEMM phase
+      if(ncc == 1) hb_phase_mark(c, HB_PH_OZ_SLICE);
+      HB_CHECK(hb_ws_reserve(c, sizeof(double) * (size_t)st.n_items * TM * TN));
+      if(c->timing && ncc == 1) HB_CUDA(cudaEventRecord(c->ev_syrk0, c->stream));
+    }
+    const OzItem* items = st.d_items + (q == ncc - 1 ? st.n_items : 0);
+    if(S == 6) HB_CHECK(launch_gemm<6>(c, st, items, chunk_stages, q > 0, (double*)c->ws));
+    else if(S == 7) HB_CHECK(launch_gemm<7>(c, st, items, chunk_stages, q > 0, (double*)c->ws));
+    else HB_CHECK(launch_gemm<8>(c, st, items, chunk_stages, q > 0, (double*)c->ws));
+  }
   if(c->timing) {
     HB_CUDA(cudaEventRecord(c->ev_syrk1, c->stream));
     c->syrk_timed = true;

@@ -93,6 +93,11 @@ class Context:
         check(self.L.hb_ctx_last_syrk_ms(self.h, ctypes.byref(ms)), "hb_ctx_last_syrk_ms")
         return float(ms.value)
 
+    def set_oz_workspace_limit(self, nbytes: int):
+        """Bound on the int8 slice buffer of the condensation (0 = AUTO: free device memory minus 1 GiB). Above the bound the columns
+        are sliced and multiplied in chunks; a buffer held above it is released now. See include/hiopb200.h."""
+        check(self.L.hb_ctx_set_oz_workspace_limit(self.h, int(nbytes)), "hb_ctx_set_oz_workspace_limit")
+
     def launch_count(self) -> int:
         return int(self.L.hb_launch_count())
 
@@ -358,6 +363,10 @@ class KKTLinSysLowRank:
 
     def fallback_count(self) -> int:
         return int(self.ctx.L.hb_lowrank_fallback_count(self.h))
+
+    def condense_chunks(self) -> int:
+        """column chunks of the last int8-slice condensation: 1 = unchunked, 0 = the FP64 kernel ran"""
+        return int(self.ctx.L.hb_lowrank_last_condense_chunks(self.h))
 
     def solveCompressed(self, rx, ryc, ryd, dx, dyc, dyd) -> bool:
         """rx is clobbered, like in the reference (hiopKKTLinSys.cpp:1178)."""

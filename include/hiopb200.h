@@ -56,13 +56,15 @@ void* hb_ctx_stream(hb_ctx* ctx);
 int hb_ctx_device(hb_ctx* ctx);
 
 /* Kernel-level timing for roofline reporting: when enabled, CUDA events bracket the dominant kernel of the condensation -- whichever
- * ran: the FP64 DMMA SYRK (k_syrk_ws) or the int8-slice tcgen05 GEMM (k_oz_gemm) -- on the context stream; hb_ctx_last_syrk_ms waits
- * for it and returns its device duration. */
+ * ran: the FP64 DMMA SYRK (k_syrk_ws) or the int8-slice tcgen05 GEMM (k_oz_gemm; with column chunks, the slicing and GEMMs of all
+ * chunks) -- on the context stream; hb_ctx_last_syrk_ms waits for it and returns its device duration. */
 int hb_ctx_enable_timing(hb_ctx* ctx, int on);
 /* Per-phase timeline of one quasi-Newton step (per-rank evidence for the multi-GPU runs): hb_ctx_phase_timeline(ctx, 1, NULL) arms the
  * marks, the next hb_lowrank_update + condense + solve_compressed records an event after each phase, hb_ctx_phase_timeline(ctx, 0, ms)
  * returns 12 durations in ms: update, row maxima (+ fused row dots), slicing, GEMM + fix-up (the whole condensation with the FP64 kernel),
- * all-reduce, V/U/N assembly, Cholesky, H^-1 rx, J dx (+ all-reduce), SPD solve, J^T dy, H^-1 rx (second). */
+ * all-reduce, V/U/N assembly, Cholesky, H^-1 rx, J dx (+ all-reduce), SPD solve, J^T dy, H^-1 rx (second). With an int8-slice
+ * condensation in several column chunks (hb_lowrank_last_condense_chunks > 1) the slicing entry is 0 and the GEMM entry holds the
+ * slicing and GEMM of every chunk. */
 int hb_ctx_phase_timeline(hb_ctx* ctx, int on, float* ms_host10);
 int hb_ctx_last_syrk_ms(hb_ctx* ctx, float* ms_host);
 
@@ -282,9 +284,21 @@ int hb_lowrank_condense(hb_lowrank* k);
 #define HB_CONDENSE_AUTO (-1)      /* default: 8 slices on tcgen05 when the GLOBAL n (summed over the ranks) >= 32768 and m+2l >= 64, FP64 DMMA otherwise */
 #define HB_CONDENSE_FP64_DMMA 0
 int hb_lowrank_set_condense_mode(hb_lowrank* k, int mode);
+/* Memory of the int8-slice modes. The slices of all n_local columns take S * Mpad * Kpad bytes (Mpad = m+2l rounded up to 128, Kpad =
+ * n_local rounded up to 128): as much as the Jacobian in FP64 at S = 8. The context allocates them once when they fit its budget; otherwise
+ * it slices and multiplies the columns in chunks of a whole number of int32-safe recombination chunks (65 408 columns at S = 8, 74 880 at
+ * S = 7, 87 296 at S = 6) through one buffer of S * Mpad * chunk bytes. The digits are the same either way (row exponents come from all
+ * columns); only the grouping of the FP64 partial sums differs, at rounding level.
+ * The budget: hb_ctx_set_oz_workspace_limit(ctx, bytes), or the environment variable HB_OZ_WORKSPACE_MB read when the context is created;
+ * 0 (the default) = AUTO: the free device memory minus 1 GiB, plus the slice buffer already held. Setting a limit below the buffer held
+ * releases it. When not even one recombination chunk (or all columns, when fewer) fits, HB_CONDENSE_AUTO redoes the condensation with the
+ * FP64 kernel (counted by hb_lowrank_fallback_count); an explicit 6/7/8 mode fails with HB_ERR_ALLOC.
+ * hb_lowrank_last_condense_chunks: column chunks of the last condensation, 1 = unchunked, 0 = the FP64 kernel ran. */
+int hb_ctx_set_oz_workspace_limit(hb_ctx* ctx, size_t bytes);
+int hb_lowrank_last_condense_chunks(hb_lowrank* k);
 /* hb_lowrank_condense is synchronous: it returns HB_ERR_NUMERIC when V is singular or N is not numerically SPD. In AUTO mode an
- * int8-slice condensation whose Cholesky breaks down is first redone with the exact FP64 kernel (hb_lowrank_fallback_count counts
- * these). hb_lowrank_condense_async only enqueues the work (no host synchronisation; this is also what an implicit condensation
+ * int8-slice condensation whose Cholesky breaks down, or whose slices do not fit (above), is first redone with the exact FP64 kernel
+ * (hb_lowrank_fallback_count counts these). hb_lowrank_condense_async only enqueues the work (no host synchronisation; this is also what an implicit condensation
  * inside hb_lowrank_solve_compressed does); a breakdown is then reported by hb_lowrank_check / hb_lowrank_last_solve_stats, the next
  * calls that synchronise. */
 int hb_lowrank_condense_async(hb_lowrank* k);
